@@ -5,7 +5,7 @@
                target index build + target covariances (k=20) + source index + source covariances +
                LM align (DLO's S2M parameters: k=20, max-corr 0.5 m, 32 iterations, eps 0.01)
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 `value`  : scan pairs per second, inputs already resident in HBM (device pointers into the C ABI)
 `e2e`    : same through the public API with pinned HOST buffers (H2D of both clouds and D2H of the result inside the
@@ -13,6 +13,8 @@
 `roofline`: dominant kernel group (exact kNN + covariance over the 500k submap) — algorithmic 64 B/point / its CUDA-event time
 `cpu_baseline`: the CPU oracle (reference's vendored nanoflann + restated GICP math, OpenMP) on this host's cores
 --impl reference: that CPU path alone, same workload/metric.
+--dump-outputs DIR: after the timed steps, what the last one computed goes to DIR/<name>.npy (see dump_outputs), so that
+two builds can be compared output for output on the same seeded inputs.
 N>1: one process per GPU (torchrun), every rank registers its own scans against the submap (weak scaling), no collective
 on the data path; barrier + max-over-ranks timing.
 """
@@ -22,6 +24,7 @@ import argparse
 import json
 import os
 import sys
+import tempfile
 import threading
 import time
 
@@ -37,7 +40,10 @@ SUBMAP_POINTS = 500_000
 KEYFRAME_STRIDE = 33                                         # 5 m at 0.15 m per scan (threshD, cfg/params.yaml:40)
 SRC_INDEX = 12 * KEYFRAME_STRIDE + 10
 SRC_LEAF = 0.27
-CACHE = os.environ.get("NGICP_BENCH_CACHE", os.path.join(ROOT, ".bench_cache", "c2_v2.npz"))
+# generated inputs are cached outside the checkout, which may be read-only; per user, so nobody else's file is read
+CACHE = os.environ.get("NGICP_BENCH_CACHE",
+                       os.path.join(tempfile.gettempdir(), f"ngicp_bench_cache_{os.getuid()}", "c2_v2.npz"))
+DUMP_TARGET_COV_ROWS = 1 << 16     # --dump-outputs: seeded sample of the 500k target covariances (8 MiB instead of 64)
 
 
 def make_workload(voxel_filter, log=lambda *a: None):
@@ -181,6 +187,23 @@ def gpu_step(g, submap, scan, guess):
     return g.result
 
 
+def dump_outputs(out_dir, g):
+    """What a caller of gpu_step receives from its last call, as .npy files: the registration result (float32 transform,
+    float64 state / Hessian / LM values, counts as float64) and the covariances of both clouds, the target's as a fixed
+    seeded sample of rows."""
+    r = g.result
+    tc = g.getTargetCovariances()
+    rows = np.sort(np.random.default_rng(0).choice(tc.shape[0], min(DUMP_TARGET_COV_ROWS, tc.shape[0]), replace=False))
+    arrays = {"final_transformation": g.getFinalTransformation(), "final_state": g.final_state(),
+              "final_hessian": g.getFinalHessian(), "lm_lambda_last_error": np.array([r.lm_lambda, r.last_error]),
+              "counts": np.array([r.nr_iterations, r.converged, r.n_linearize, r.n_compute_error, r.lm_failed], np.float64),
+              "source_covariances": g.getSourceCovariances(),
+              "target_covariances_sample": tc[rows], "target_covariances_sample_rows": rows.astype(np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -194,7 +217,12 @@ def main():
                     "(5M-point submap sharded over the ranks, fused NVLink exchange) and report them as sub-objects")
     ap.add_argument("--c4-pairs", type=int, default=10000)
     ap.add_argument("--c5-target", type=int, default=5_000_000)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what rank 0's last timed GPU step computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the GPU path's outputs; it does not apply to --impl reference")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -293,6 +321,8 @@ def main():
         barrier()
         t_wall = time.perf_counter() - t_wall0
     launches = (L.ngicp_launch_count() - launches0)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, g)      # before the end-to-end steps below overwrite the handle's results
     grids = {"target": g.grid_info(1), "source": g.grid_info(0)}
     # end to end: pinned host buffers in, result struct out, every step
     for _ in range(2):
@@ -394,7 +424,7 @@ def main():
         try:
             # the scan's k=20 covariances are split over the ranks + one all-reduce when there is more than one
             # (2 GPUs: 3.72 -> 3.63 ms/scan; the replicated covariances are the largest non-align item at 8)
-            c5 = bc.c5_bench(local_rank, rank, world, target_points=args.c5_target, steps=10, check=1,
+            c5 = bc.c5_bench(local_rank, rank, world, target_points=args.c5_target, steps=args.steps, check=1,
                              shard_source_covs=1 if world > 1 else 0)
         except Exception as e:
             c5 = {"error": repr(e)}

@@ -22,6 +22,7 @@ import argparse
 import json
 import os
 import sys
+import tempfile
 import time
 from concurrent.futures import ProcessPoolExecutor, ThreadPoolExecutor
 
@@ -584,7 +585,8 @@ def _gen_dense(i):
 
 
 def c5_workload(n_target, log):
-    cache = os.path.join(ROOT, ".bench_cache", f"c5_v2_{n_target}.npz")
+    # outside the checkout, which may be read-only; per user, so nobody else's file is read
+    cache = os.path.join(tempfile.gettempdir(), f"ngicp_bench_cache_{os.getuid()}", f"c5_v2_{n_target}.npz")
     if os.path.exists(cache):
         z = np.load(cache)
         return {k: z[k] for k in z.files}
