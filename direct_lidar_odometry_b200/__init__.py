@@ -9,11 +9,11 @@ The compute lives in csrc/ (hand-written CUDA behind the C ABI of include/nanogi
 from . import synth  # noqa: F401  (pure numpy)
 from . import pointcloud2  # noqa: F401  (plain data + field mapping, no ROS)
 
-__all__ = ["NanoGICP", "NanoGICPError", "CovarianceView", "KeyframeStore", "align_batch", "imu_prior", "synth", "pointcloud2", "lib_path"]
+__all__ = ["NanoGICP", "NanoGICPError", "CovarianceView", "KeyframeStore", "align_batch", "fitness_batch", "imu_prior", "synth", "pointcloud2", "lib_path"]
 
 
 def __getattr__(name):
-    if name in ("NanoGICP", "NanoGICPError", "CovarianceView", "KeyframeStore", "align_batch", "imu_prior"):
+    if name in ("NanoGICP", "NanoGICPError", "CovarianceView", "KeyframeStore", "align_batch", "fitness_batch", "imu_prior"):
         from . import nanogicp
         return getattr(nanogicp, name)
     if name == "lib_path":

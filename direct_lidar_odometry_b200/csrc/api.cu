@@ -50,6 +50,10 @@ struct ngicp_handle {
   bool comm_peer_ipc[NGICP_MAX_RANKS] = {};
   PeerComm comm;
   bool comm_on = false;
+  // results of ngicp_fitness_batch when this handle leads the batch: pinned + mapped, written by the finalize kernel
+  FitnessResult* fit_pinned = nullptr;
+  FitnessResult* fit_mapped = nullptr;
+  size_t fit_cap = 0;
 };
 
 // N1: device-resident keyframe store (SURVEY §8f).  A keyframe is the pair DLO keeps on the host — the voxelised
@@ -553,6 +557,7 @@ void ngicp_destroy(ngicp_t* h) {
   if (h->comm_buf) cudaFree(h->comm_buf);
   if (h->res_pinned) cudaFreeHost(h->res_pinned);
   if (h->red_pinned) cudaFreeHost(h->red_pinned);
+  if (h->fit_pinned) cudaFreeHost(h->fit_pinned);
   for (int i = 0; i < PH_COUNT; i++)
     for (int j = 0; j < 2; j++)
       if (h->ev[i][j]) cudaEventDestroy(h->ev[i][j]);
@@ -819,6 +824,82 @@ int ngicp_transform_source(ngicp_t* h, const float* T16, float* out_xyz1, size_t
   NG_CUDA(h, cudaMemcpyAsync(out_xyz1, h->sc.queries.p, sizeof(float4) * n, cudaMemcpyDefault, h->stream->s));
   NG_CUDA(h, cudaStreamSynchronize(h->stream->s));
   return NGICP_OK;
+}
+
+// pcl::Registration::getFitnessScore for n handles, each with its own source, target and T (fitness.cu): the handles'
+// streams are joined into the first one's, which runs the two launches and lands the results in its mapped host buffer.
+// The registration state (correspondences, lin_valid, results) is left alone.
+int ngicp_fitness_batch(ngicp_t* const* hs, size_t n, const float* T16s, double max_range, double* scores, size_t* n_inliers) {
+  if (!hs || n == 0 || !hs[0]) return NGICP_E_INVALID;
+  ngicp_t* h0 = hs[0];
+  if (!T16s || !scores) return fail(h0, NGICP_E_INVALID, "fitness: null argument");
+  if (std::isnan(max_range)) return fail(h0, NGICP_E_INVALID, "fitness: max_range is NaN");
+  if (n > 0x7fffffffu) return fail(h0, NGICP_E_INVALID, "fitness: too many handles");
+  for (size_t i = 0; i < n; ++i) {
+    ngicp_t* h = hs[i];
+    if (!h) return fail(h0, NGICP_E_INVALID, "fitness: null handle");
+    if (h->device != h0->device) return fail(h0, NGICP_E_INVALID, "fitness: handles live on different devices");
+    for (size_t j = 0; j < i; ++j)
+      if (hs[j] == h) return fail(h0, NGICP_E_INVALID, "fitness: the same handle appears twice");
+    const std::string pre = n > 1 ? "fitness: pair " + std::to_string(i) + ": " : "fitness: ";
+    // a sharded handle holds one slab of the submap: its nearest neighbours are not the submap's
+    if (h->comm_on || h->slab_axis >= 0) return fail(h0, NGICP_E_UNSUPPORTED, (pre + "handle is in sharded mode").c_str());
+    if (!h->src || !h->tgt) return fail(h0, NGICP_E_STATE, (pre + "source/target not set").c_str());
+    if (h->tgt->n > 0 && !h->tgt->indexed) return fail(h0, NGICP_E_STATE, (pre + "target has no search index").c_str());
+  }
+  DeviceGuard g(h0->device);
+  std::vector<FitnessPair> pairs(n);
+  long long chunks = 0;
+  for (size_t i = 0; i < n; ++i) {
+    ngicp_t* h = hs[i];
+    join_source(h);   // the source was uploaded on the source-side stream
+    if (h != h0) {    // everything queued on this handle's stream (target index) precedes the launches
+      if (!h->sc.copy_done) NG_CUDA(h0, cudaEventCreateWithFlags(&h->sc.copy_done, cudaEventDisableTiming));
+      NG_CUDA(h0, cudaEventRecord(h->sc.copy_done, h->stream->s));
+      NG_CUDA(h0, cudaStreamWaitEvent(h0->stream->s, h->sc.copy_done, 0));
+    }
+    FitnessPair& p = pairs[i];
+    memset(&p, 0, sizeof p);
+    const float* T = T16s + 16 * i;   // column-major: (r,c) at [c*4+r]
+    for (int r = 0; r < 3; ++r)
+      for (int c = 0; c < 4; ++c) p.T[r * 4 + c] = T[c * 4 + r];
+    p.src = h->src->pts.as<float4>();
+    p.ns = h->src->n;
+    p.chunk0 = (int)chunks;
+    if (h->src->n > 0 && h->tgt->n > 0) {
+      p.tgt = h->tgt->view();
+      p.nchunks = (h->src->n + FITNESS_CHUNK - 1) / FITNESS_CHUNK;
+      // two lanes per point against a target much larger than the scan (the registration kernels' rule)
+      p.lpp = (long long)h->tgt->n >= 4ll * h->src->n ? 2 : 1;
+    }
+    chunks += p.nchunks;
+  }
+  if (chunks > 0x7fffffff) return fail(h0, NGICP_E_INVALID, "fitness: too many source points");
+  if (h0->fit_cap < n) {
+    if (h0->fit_pinned) cudaFreeHost(h0->fit_pinned);
+    h0->fit_pinned = h0->fit_mapped = nullptr;
+    h0->fit_cap = 0;
+    NG_CUDA(h0, cudaHostAlloc((void**)&h0->fit_pinned, sizeof(FitnessResult) * n, cudaHostAllocMapped));
+    NG_CUDA(h0, cudaHostGetDevicePointer((void**)&h0->fit_mapped, h0->fit_pinned, 0));
+    h0->fit_cap = n;
+  }
+  Scratch& sc = h0->sc;
+  NG_CUDA(h0, sc.fit_args.reserve(sizeof(FitnessPair) * n, h0->stream));
+  NG_CUDA(h0, sc.fit_partials.reserve(sizeof(double2) * (size_t)(chunks > 0 ? chunks : 1), h0->stream));
+  NG_CUDA(h0, cudaMemcpyAsync(sc.fit_args.p, pairs.data(), sizeof(FitnessPair) * n, cudaMemcpyHostToDevice, h0->stream->s));
+  NG_CUDA(h0, launch_fitness(sc.fit_args.as<FitnessPair>(), (int)n, (int)chunks, max_range, sc.fit_partials.as<double2>(), h0->fit_mapped,
+                             h0->stream->s));
+  NG_CUDA(h0, cudaStreamSynchronize(h0->stream->s));
+  for (size_t i = 0; i < n; ++i) {
+    scores[i] = h0->fit_pinned[i].score;
+    if (n_inliers) n_inliers[i] = (size_t)h0->fit_pinned[i].n;
+  }
+  return NGICP_OK;
+}
+
+int ngicp_fitness_score(ngicp_t* h, const float* T16, double max_range, double* score, size_t* n_inliers) {
+  if (!h) return NGICP_E_INVALID;
+  return ngicp_fitness_batch(&h, 1, T16, max_range, score, n_inliers);
 }
 
 int ngicp_voxel_filter(ngicp_t* h, const void* in, size_t n, size_t stride, float leaf, void* out, size_t cap, size_t* m) {

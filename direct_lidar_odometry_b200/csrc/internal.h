@@ -137,6 +137,7 @@ struct Scratch {
   DevBuf barrier;    // unsigned counters for the grid barrier
   DevBuf trace;      // debug: %globaltimer stamps of the fused kernel
   DevBuf batch_args; // BatchPair records of ngicp_align_batch
+  DevBuf fit_args, fit_partials;   // FitnessPair records and per-chunk {sum, count} of ngicp_fitness_batch
 };
 
 // number of kernels launched by this library since load (diagnostics; ngicp_launch_count())
@@ -210,6 +211,22 @@ void align_prime_kernels(int device);
 void knn_prime_kernels();
 void voxel_prime_kernels();
 void index_prime_kernels();
+
+// ---- fitness.cu -----------------------------------------------------------------------------------
+// pcl::Registration::getFitnessScore over n pairs (ngicp_fitness_score / ngicp_fitness_batch), two launches in all
+constexpr int FITNESS_CHUNK = 256;   // source points per work item: fixed, so a pair's summation order never changes
+struct FitnessPair {
+  const float4* src; int ns;
+  GridView tgt;
+  float T[12];      // rows of the float transform: T[r*4+c], c = 3 the translation
+  int lpp;          // lanes per source point in the radius-1 cube search (1 or 2)
+  int chunk0;       // first chunk of this pair in the launch
+  int nchunks;      // 0 for an empty source or target
+};
+struct FitnessResult { double score; unsigned long long n; };
+// partials: double2[total_chunks]; out: n_pairs results (mapped host memory)
+cudaError_t launch_fitness(const FitnessPair* pairs_dev, int n_pairs, int total_chunks, double max_range, double2* partials,
+                           FitnessResult* out, cudaStream_t st);
 
 // ---- voxel.cu -------------------------------------------------------------------------------------
 // returns cudaSuccess; *m_out and *overflow are valid after the call (it synchronises once to learn m)

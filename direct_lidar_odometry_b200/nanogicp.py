@@ -361,6 +361,21 @@ class NanoGICP:
     def getFinalTransformation(self) -> np.ndarray:
         return self._final.copy()
 
+    def getFitnessScore(self, max_range: float = sys.float_info.max, T=None) -> float:
+        """pcl::Registration::getFitnessScore(max_range): the mean SQUARED distance from the source, transformed by T
+        (default: getFinalTransformation()), to its nearest target point, over the points whose squared distance is
+        <= max_range (PCL compares the squared distance with max_range as given).  sys.float_info.max when no point
+        qualifies.  Searches the device index, so it also works on a target set by KeyframeStore.set_target."""
+        return self.fitness(T, max_range)[0]
+
+    def fitness(self, T=None, max_range: float = sys.float_info.max):
+        """(score, number of points that entered it) of getFitnessScore — ngicp_fitness_score."""
+        Tf = _mat_to_abi(self._final if T is None else T, np.float32)
+        score, n = C.c_double(0), C.c_size_t(0)
+        self._check(self._L.ngicp_fitness_score(self._h, Tf.ctypes.data_as(C.POINTER(C.c_float)), float(max_range),
+                                                C.byref(score), C.byref(n)))
+        return score.value, int(n.value)
+
     def hasConverged(self) -> bool:
         return self._converged
 
@@ -643,6 +658,28 @@ def align_batch(handles, guesses=None):
         h.nr_iterations_ = int(h._res.nr_iterations)
         out.append(h._res)
     return out
+
+
+def fitness_batch(handles, transforms=None, max_range: float = sys.float_info.max):
+    """ngicp_fitness_batch: getFitnessScore(max_range) of len(handles) independent pairs (each NanoGICP object with its
+    own source and target) in a constant number of launches, bit-identical to the single calls.  transforms: sequence
+    of 4x4 matrices (None entries = that handle's getFinalTransformation()) or None.  Returns (scores, counts) as
+    float64 / int64 arrays."""
+    n = len(handles)
+    if n == 0:
+        return np.zeros(0), np.zeros(0, dtype=np.int64)
+    L = handles[0]._L
+    arr = (C.c_void_p * n)(*[h._h for h in handles])
+    ta = np.zeros((n, 16), dtype=np.float32)
+    for i, h in enumerate(handles):
+        T = None if transforms is None else transforms[i]
+        ta[i] = _mat_to_abi(h._final if T is None else T, np.float32)
+    scores = np.zeros(n)
+    counts = np.zeros(n, dtype=np.uint64)
+    handles[0]._check(L.ngicp_fitness_batch(arr, n, ta.ctypes.data_as(C.POINTER(C.c_float)), float(max_range),
+                                            scores.ctypes.data_as(C.POINTER(C.c_double)),
+                                            counts.ctypes.data_as(C.POINTER(C.c_size_t))))
+    return scores, counts.astype(np.int64)
 
 
 class KeyframeStore:

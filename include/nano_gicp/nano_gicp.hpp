@@ -17,6 +17,7 @@
 #include <cfloat>
 #include <cstdio>
 #include <cstring>
+#include <limits>
 #include <memory>
 #include <stdexcept>
 #include <string>
@@ -323,6 +324,22 @@ class NanoGICP {
     }
   }
   Matrix4 getFinalTransformation() const { return final_transformation_; }
+  // pcl::Registration::getFitnessScore(max_range): the mean squared distance from the source, transformed by
+  // final_transformation_ (in float, as pcl::transformPointCloud), to its nearest target point, over the points whose
+  // SQUARED distance is <= max_range — PCL compares the squared distance with max_range as given.  DBL_MAX when no point
+  // qualifies.  PCL searches its own tree_, which DLO never builds (it calls setSearchMethodTarget(null, true)); this
+  // version searches the handle's device index, so it works in every configuration, also after
+  // KeyframeStore::setTarget.  A missing source, target or index prints and returns DBL_MAX; CUDA errors throw.
+  double getFitnessScore(double max_range = std::numeric_limits<double>::max()) {
+    double score = DBL_MAX;
+    const int rc = ngicp_fitness_score(h(), final_transformation_.data(), max_range, &score, nullptr);
+    if (rc == NGICP_E_STATE) {
+      std::fprintf(stderr, "[pcl::Registration::getFitnessScore] %s\n", ngicp_last_error(h()));
+      return DBL_MAX;
+    }
+    if (rc < 0) throw std::runtime_error(std::string("NanoGICP-B200: getFitnessScore failed: ") + (h() ? ngicp_last_error(h()) : "no handle"));
+    return score;
+  }
   bool hasConverged() const { return converged_; }
   const ngicp_result& getLastResult() const { return last_result_; }
 

@@ -190,6 +190,16 @@ int ngicp_align_batch(ngicp_t* const* handles, size_t n, const float* guesses16,
 /* pcl::transformPointCloud(*input_, output, final) at lsq_registration_impl.hpp:114: writes n packed
  * {x,y,z,1} float4 records (host or device); the facade merges them into the output cloud's records */
 int ngicp_transform_source(ngicp_t* h, const float* T16, float* out_xyz1, size_t n);
+/* pcl::Registration::getFitnessScore(max_range): mean squared distance from the source, transformed by T (float,
+ * column-major, as pcl::transformPointCloud), to its nearest target point, over the points whose SQUARED distance is
+ * <= max_range (PCL's comparison).  *score = DBL_MAX and *n_inliers = 0 when no point qualifies.  n_inliers may be NULL.
+ * Empty source or target: DBL_MAX / 0.  NGICP_E_INVALID: null arguments or a NaN max_range; NGICP_E_STATE: no source, no
+ * target, or a target without a search index; NGICP_E_UNSUPPORTED: a handle in sharded mode (it holds one slab of the
+ * target).  Touches no registration state. */
+int ngicp_fitness_score(ngicp_t* h, const float* T16, double max_range, double* score, size_t* n_inliers);
+/* the same for n handles (own source + target each, one device, each at most once) in a constant number of launches;
+ * T16s: n x 16 floats; bit-identical to n single calls */
+int ngicp_fitness_batch(ngicp_t* const* handles, size_t n, const float* T16s, double max_range, double* scores, size_t* n_inliers);
 
 /* ---- voxel grid ------------------------------------------------------------------------------- */
 /* pcl::VoxelGrid<PointXYZI>::filter with leaf (l,l,l) (odom.cc:126-127,460-463,487-490,1160-1163).
