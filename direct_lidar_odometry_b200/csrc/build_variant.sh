@@ -7,6 +7,6 @@ mkdir -p variants
 NVCC=${NVCC:-/usr/local/cuda/bin/nvcc}
 ARCH="-gencode arch=compute_100a,code=sm_100a"
 $NVCC -O3 -std=c++17 $ARCH -lineinfo -Xcompiler -fPIC --expt-relaxed-constexpr -ccbin /usr/bin/g++ -fmad=false $2 -c knn_cov.cu -o variants/knn_cov_$1.o
-$NVCC $ARCH -shared -cudart static -o variants/libnanogicp_$1.so sort_scan.o cloud_index.o variants/knn_cov_$1.o align.o voxel.o api.o submap_select.o
+$NVCC $ARCH -shared -cudart static -o variants/libnanogicp_$1.so sort_scan.o cloud_index.o variants/knn_cov_$1.o align.o voxel.o fitness.o api.o submap_select.o
 rm -f variants/knn_cov_$1.o
 echo built variants/libnanogicp_$1.so

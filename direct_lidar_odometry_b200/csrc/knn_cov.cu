@@ -1196,6 +1196,24 @@ cudaError_t launch_covariances(const DevCloud& c, int k, int method, int* nbr_sc
         fprintf(stderr, "[ngicp knn]   tile kernel: %llu warps, span %.1f us, mean warp busy %.1f us (%.0f%% of the span)\n", h[ST_TWARPS],
                 1e-3 * (double)(h[ST_TEND] - h[ST_TSTART]), 1e-3 * (double)h[ST_TSUM] / (double)h[ST_TWARPS],
                 100.0 * (double)h[ST_TSUM] / (double)h[ST_TWARPS] / (double)(h[ST_TEND] - h[ST_TSTART]));
+      // the control words of the plan / tile / rest launches, and the plan's work items by box edge (how far it split)
+      int hc[CT_N] = {};
+      cudaMemcpyAsync(hc, ctrl, sizeof(hc), cudaMemcpyDeviceToHost, st);
+      cudaStreamSynchronize(st);
+      const int nslow = hc[CT_SLOW], nall = nslow + hc[CT_ITEMS];
+      long long by_edge[3] = {0, 0, 0};      // box edge TQ_CORE, TQ_CORE / 2, 1 cells
+      if (nall > 0 && nall <= c.n) {
+        int4* hi = static_cast<int4*>(malloc(sizeof(int4) * (size_t)c.n));
+        if (hi != nullptr && cudaMemcpy(hi, items, sizeof(int4) * (size_t)c.n, cudaMemcpyDeviceToHost) == cudaSuccess) {
+          for (int w = 0; w < nall; ++w) {
+            const int sz = hi[w < nslow ? w : c.n - 1 - (w - nslow)].w & 255;
+            by_edge[sz == TQ_CORE ? 0 : (sz == 1 ? 2 : 1)]++;
+          }
+        }
+        free(hi);
+      }
+      fprintf(stderr, "[ngicp knn]   control: rest=%d fix=%d slow=%d items=%d, items by box edge %d / %d / 1: %lld / %lld / %lld\n",
+              hc[CT_REST], hc[CT_FIX], nslow, hc[CT_ITEMS], TQ_CORE, TQ_CORE / 2, by_edge[0], by_edge[1], by_edge[2]);
     }
     launch_cov_kernel(c, k, method, nbr_scratch, covs6, q_lo, q_hi, fb_flags, nullptr, nullptr, st, k == 10 || k == 20);
     if (overlap && (e = cudaStreamWaitEvent(st, side->join, 0)) != cudaSuccess) return e;

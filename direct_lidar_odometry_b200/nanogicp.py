@@ -401,7 +401,8 @@ class NanoGICP:
 
     def cov_neighbors(self, which: int):
         """(idx (n,k) original indices, d2 (n,k)) of the neighbours the last calculate*Covariances call on this handle
-        summed over, in summation order (ascending distance, ties by index) — ngicp_cov_neighbors."""
+        summed over, in summation order — ngicp_cov_neighbors.  The order is ascending squared distance; exact ties are
+        broken by sorted slot, i.e. by (grid cell, original index), not by original index alone."""
         n = int(self._L.ngicp_cloud_size(self._h, which))
         k = int(self._p.k_correspondences)
         idx = np.zeros((n, k), dtype=np.int32)
