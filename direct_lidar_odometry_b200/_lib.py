@@ -29,7 +29,7 @@ EXPORTS = [
     "ngicp_version", "ngicp_launch_count", "ngicp_grid_info", "ngicp_set_owner_slab", "ngicp_lm_trial",
     "ngicp_lm_is_converged", "ngicp_comm_export", "ngicp_comm_connect", "ngicp_comm_connect_local", "ngicp_comm_close", "ngicp_comm_reset", "ngicp_preprocess", "ngicp_preprocess_pointcloud2", "ngicp_calc_source_covs_part", "ngicp_covs_device", "ngicp_transform_voxel_filter", "ngicp_kfstore_create", "ngicp_kfstore_destroy", "ngicp_kfstore_size",
     "ngicp_kfstore_points", "ngicp_kfstore_push", "ngicp_kfstore_set_target", "ngicp_cov_neighbors", "ngicp_align_batch", "ngicp_imu_prior",
-    "ngicp_nn1_packed", "ngicp_linearize_won", "ngicp_fitness_score", "ngicp_fitness_batch",
+    "ngicp_nn1_packed", "ngicp_linearize_won", "ngicp_fitness_score", "ngicp_fitness_batch", "ngicp_correspondences",
     "ngicp_submap_push_indices", "ngicp_submap_convex_hull", "ngicp_submap_concave_hull", "ngicp_submap_selector_create",
     "ngicp_submap_selector_destroy", "ngicp_submap_select", "ngicp_submap_selector_hulls", "ngicp_keyframe_wanted",
 ]
@@ -113,6 +113,7 @@ def load() -> C.CDLL:
     proto("ngicp_knn", i32, vp, i32, vp, sz, sz, i32, ip, fp)
     proto("ngicp_cov_neighbors", i32, vp, i32, ip, fp)
     proto("ngicp_linearize", i32, vp, dp, dp, dp, dp, ip, fp, dp)
+    proto("ngicp_correspondences", i32, vp, ip, fp, dp)
     proto("ngicp_compute_error", i32, vp, dp, dp)
     proto("ngicp_linearize_partial", i32, vp, dp, vp)
     proto("ngicp_nn1_packed", i32, vp, dp, C.c_uint, vp)

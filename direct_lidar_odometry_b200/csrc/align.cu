@@ -96,7 +96,8 @@ __device__ __forceinline__ void finish_point(const AlignArgs& a, const Iso3& Td,
     a.tgt_pt[i] = tp;
   }
   a.corr[i] = corr;
-  a.sqd[i] = my_d;
+  // without a correspondence the search may have stopped at the cap with any candidate: report none, not that one
+  a.sqd[i] = corr >= 0 ? my_d : FLT_MAX;
 }
 
 __device__ __forceinline__ double error_point(const AlignArgs& a, const Iso3& Td, int i) {

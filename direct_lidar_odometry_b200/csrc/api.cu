@@ -1113,6 +1113,25 @@ int ngicp_linearize(ngicp_t* h, const double* T16, double* H36, double* b6, doub
   return NGICP_OK;
 }
 
+int ngicp_correspondences(ngicp_t* h, int* corr, float* sqd, double* mahal16) {
+  if (!h) return NGICP_E_INVALID;
+  if (!h->lin_valid || !h->src) return fail(h, NGICP_E_STATE, "correspondences: no linearisation on the current clouds");
+  DeviceGuard g(h->device);
+  const size_t ns = (size_t)h->src->n;
+  if (corr) NG_CUDA(h, cudaMemcpyAsync(corr, h->sc.corr.p, sizeof(int) * ns, cudaMemcpyDefault, h->stream->s));
+  if (sqd) NG_CUDA(h, cudaMemcpyAsync(sqd, h->sc.sqd.p, sizeof(float) * ns, cudaMemcpyDefault, h->stream->s));
+  if (mahal16) {
+    AlignBuffers ab;
+    memset(&ab, 0, sizeof ab);
+    ab.ns = (int)ns; ab.mahal = h->sc.mahal.as<double>(); ab.corr = h->sc.corr.as<int>();
+    NG_CUDA(h, h->sc.cov_stage.reserve(sizeof(double) * 16 * ns, h->stream));
+    NG_CUDA(h, launch_export_mahal(ab, h->sc.cov_stage.as<double>(), h->stream->s));
+    NG_CUDA(h, cudaMemcpyAsync(mahal16, h->sc.cov_stage.p, sizeof(double) * 16 * ns, cudaMemcpyDefault, h->stream->s));
+  }
+  NG_CUDA(h, cudaStreamSynchronize(h->stream->s));
+  return NGICP_OK;
+}
+
 int ngicp_compute_error_partial(ngicp_t* h, const double* T16, double* out1) {
   if (!h || !T16 || !out1) return NGICP_E_INVALID;
   if (!h->lin_valid) return fail(h, NGICP_E_STATE, "compute_error needs a preceding linearize on the same clouds");

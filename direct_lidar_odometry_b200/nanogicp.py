@@ -428,6 +428,19 @@ class NanoGICP:
             out["mahalanobis"] = mah.reshape(n, 4, 4).transpose(0, 2, 1).copy()
         return out
 
+    def correspondences(self):
+        """The per-point state of the last linearisation on this handle (linearize, align or align_batch), in
+        linearize's per-point layout: dict(corr, sqd, mahalanobis (n,4,4)) — ngicp_correspondences.  After
+        align() with setMaximumIterations(1) it is the fused kernel's linearisation at the guess."""
+        n = int(self._L.ngicp_cloud_size(self._h, _lib.SOURCE))
+        corr = np.zeros(n, dtype=np.int32)
+        sqd = np.zeros(n, dtype=np.float32)
+        mah = np.zeros((n, 16))
+        self._check(self._L.ngicp_correspondences(self._h, corr.ctypes.data_as(C.POINTER(C.c_int)),
+                                                  sqd.ctypes.data_as(C.POINTER(C.c_float)),
+                                                  mah.ctypes.data_as(C.POINTER(C.c_double))))
+        return dict(corr=corr, sqd=sqd, mahalanobis=mah.reshape(n, 4, 4).transpose(0, 2, 1).copy())
+
     def compute_error(self, T) -> float:
         Tc = _mat_to_abi(T, np.float64)
         e = C.c_double(0)

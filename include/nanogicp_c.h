@@ -242,6 +242,12 @@ int ngicp_knn(ngicp_t* h, int which, const float* queries, size_t nq, size_t q_s
 /* NanoGICP::linearize (nano_gicp_impl.hpp:213-270): H 6x6 col-major, b, sum of errors; optional per-point
  * correspondences_ (target index or -1), sq_distances_, and mahalanobis_ (n*16 doubles) */
 int ngicp_linearize(ngicp_t* h, const double* T16, double* H36, double* b6, double* err, int* corr, float* sqd, double* mahal);
+/* test hook: the per-point state the LAST linearisation on this handle left behind — ngicp_linearize, a fused or stepped
+ * ngicp_align (its last linearisation; with max_iterations = 1 the one at the guess) or ngicp_align_batch — in
+ * ngicp_linearize's layout: corr[n] target index or -1, sqd[n] nearest squared distance (FLT_MAX without a
+ * correspondence), mahal16[n*16] col-major 4x4 (zero without a correspondence).  Any output may be NULL.
+ * NGICP_E_STATE when no linearisation is valid for the current clouds. */
+int ngicp_correspondences(ngicp_t* h, int* corr, float* sqd, double* mahal16);
 /* NanoGICP::compute_error (nano_gicp_impl.hpp:272-296) with the correspondences frozen by the last linearize */
 int ngicp_compute_error(ngicp_t* h, const double* T16, double* err);
 /* sharded-submap building block: like ngicp_linearize but returns the raw partial sums
