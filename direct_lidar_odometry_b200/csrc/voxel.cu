@@ -97,29 +97,55 @@ __global__ void __launch_bounds__(256) vox_pack_kernel(const unsigned char* __re
   }
 }
 
+// PCL's index-range guard (dx = (int64)((max - min) * inverse_leaf) + 1 per axis; dx*dy*dz > INT32_MAX -> warn, output =
+// input), made exact.  The cloud passes through (returns 1) wherever PCL's own arithmetic is not defined or would wrap:
+//   * an axis extent (max - min) * inv that is not finite or >= 2^31 (the int64 conversion, then dx*dy*dz, would overflow);
+//   * dx*dy*dz > INT32_MAX, computed without wrapping;
+//   * floor(min * inv) or floor(max * inv) outside int32, or div_b = max_b - min_b + 1 beyond INT32_MAX;
+//   * floor(max * inv) - (float)min_b rounding past max_b - min_b (axes wider than 2^24 cells): the last cell's index
+//     would reach div_b and alias the next row, or the invalid key;
+//   * a div_b product >= 2^32.
+// Otherwise min_b / div_b are PCL's, every float -> int conversion of the key computation is in range on any hardware,
+// every finite point's key is below div_b[0]*div_b[1]*div_b[2], and that product is the key of non-finite points.
+// SURVEY.md App. B1 states the same rule.
+__device__ int vox_grid_setup(const float lo[3], const float hi[3], float inv, int minb[3], int div[3]) {
+  long long dxyz = 1;
+  unsigned long long cells = 1;
+  for (int a = 0; a < 3; a++) { minb[a] = 0; div[a] = 1; }
+  int mnb[3], dv[3];
+  for (int a = 0; a < 3; a++) {
+    const float ext = __fmul_rn(__fsub_rn(hi[a], lo[a]), inv);
+    if (!(ext < 2147483648.f)) return 1;
+    dxyz *= (long long)ext + 1;                                   // each factor <= 2^31: no wrap before the test below
+    if (dxyz > 2147483647ll) return 1;
+    const float flo = floorf(__fmul_rn(lo[a], inv)), fhi = floorf(__fmul_rn(hi[a], inv));
+    if (!(flo >= -2147483648.f) || !(fhi < 2147483648.f)) return 1;
+    const long long span = (long long)fhi - (long long)flo;
+    if (span >= 2147483647ll || (long long)__fsub_rn(fhi, flo) > span) return 1;
+    cells *= (unsigned long long)(span + 1);
+    if (cells >= (1ull << 32)) return 1;
+    mnb[a] = (int)flo;
+    dv[a] = (int)(span + 1);
+  }
+  for (int a = 0; a < 3; a++) { minb[a] = mnb[a]; div[a] = dv[a]; }
+  return 0;
+}
+
 __global__ void vox_setup_kernel(GridDesc* d, float inv) {
   if (d->nfinite == 0) { d->voverflow = 0; for (int a = 0; a < 3; a++) { d->vmin_b[a] = 0; d->vdiv[a] = 1; } return; }
   float lo[3], hi[3];
   for (int a = 0; a < 3; a++) { lo[a] = ord2f(d->bb_min[a]); hi[a] = ord2f(d->bb_max[a]); }
-  // PCL: int64 dx = (int64)((max - min) * inverse_leaf) + 1 ...; if dx*dy*dz > INT32_MAX -> warn, output = input
-  const long long dx = (long long)(__fmul_rn(__fsub_rn(hi[0], lo[0]), inv)) + 1;
-  const long long dy = (long long)(__fmul_rn(__fsub_rn(hi[1], lo[1]), inv)) + 1;
-  const long long dz = (long long)(__fmul_rn(__fsub_rn(hi[2], lo[2]), inv)) + 1;
-  d->voverflow = (dx * dy * dz > 2147483647ll) ? 1 : 0;
-  for (int a = 0; a < 3; a++) {
-    const int mnb = (int)floorf(__fmul_rn(lo[a], inv));
-    const int mxb = (int)floorf(__fmul_rn(hi[a], inv));
-    d->vmin_b[a] = mnb;
-    d->vdiv[a] = mxb - mnb + 1;
-  }
+  int minb[3], div[3];
+  d->voverflow = vox_grid_setup(lo, hi, inv, minb, div);
+  for (int a = 0; a < 3; a++) { d->vmin_b[a] = minb[a]; d->vdiv[a] = div[a]; }
 }
 
 __global__ void __launch_bounds__(256) vox_keys_kernel(const float4* __restrict__ pts, int n, const GridDesc* __restrict__ d, float inv,
                                                        unsigned* __restrict__ keys, unsigned* __restrict__ vals) {
   const int m0 = d->vmin_b[0], m1 = d->vmin_b[1], m2 = d->vmin_b[2];
-  const int mul1 = d->vdiv[0], mul2 = d->vdiv[0] * d->vdiv[1];
+  const unsigned mul1 = (unsigned)d->vdiv[0], mul2 = (unsigned)d->vdiv[0] * (unsigned)d->vdiv[1];
   const bool bad = d->voverflow != 0;
-  const unsigned VOX_INVALID = d->voverflow ? 0u : (unsigned)(d->vdiv[0] * d->vdiv[1] * d->vdiv[2]);
+  const unsigned VOX_INVALID = d->voverflow ? 0u : (unsigned)d->vdiv[0] * (unsigned)d->vdiv[1] * (unsigned)d->vdiv[2];
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
     const float4 p = pts[i];
     unsigned key = VOX_INVALID;
@@ -127,7 +153,7 @@ __global__ void __launch_bounds__(256) vox_keys_kernel(const float4* __restrict_
       const int i0 = (int)(__fsub_rn(floorf(__fmul_rn(p.x, inv)), (float)m0));
       const int i1 = (int)(__fsub_rn(floorf(__fmul_rn(p.y, inv)), (float)m1));
       const int i2 = (int)(__fsub_rn(floorf(__fmul_rn(p.z, inv)), (float)m2));
-      key = (unsigned)(i0 + i1 * mul1 + i2 * mul2);
+      key = (unsigned)i0 + (unsigned)i1 * mul1 + (unsigned)i2 * mul2;   // < div_b product < 2^32 (vox_grid_setup)
     }
     keys[i] = key;
     vals[i] = (unsigned)i;
@@ -136,7 +162,7 @@ __global__ void __launch_bounds__(256) vox_keys_kernel(const float4* __restrict_
 
 // flags[i] = 1 at the first element of every run of equal valid keys; flags[n] = 0 (sentinel for the total)
 __global__ void __launch_bounds__(256) vox_heads_kernel(const unsigned* __restrict__ keys, int n, int* __restrict__ flags, GridDesc* __restrict__ d) {
-  const unsigned VOX_INVALID = d->voverflow ? 0u : (unsigned)(d->vdiv[0] * d->vdiv[1] * d->vdiv[2]);
+  const unsigned VOX_INVALID = d->voverflow ? 0u : (unsigned)d->vdiv[0] * (unsigned)d->vdiv[1] * (unsigned)d->vdiv[2];
   if (blockIdx.x == 0 && threadIdx.x == 0) d->n = n + 1;   // length of the scan that follows
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i <= n; i += gridDim.x * blockDim.x) {
     int f = 0;
@@ -152,7 +178,7 @@ __global__ void __launch_bounds__(256) vox_heads_kernel(const unsigned* __restri
 __global__ void __launch_bounds__(128) vox_centroid_kernel(const unsigned* __restrict__ keys, const unsigned* __restrict__ perm, int n,
                                                            const int* __restrict__ slots, const float4* __restrict__ pts,
                                                            float* __restrict__ out, int* __restrict__ slot_of_point, const GridDesc* __restrict__ d) {
-  const unsigned VOX_INVALID = d->voverflow ? 0u : (unsigned)(d->vdiv[0] * d->vdiv[1] * d->vdiv[2]);
+  const unsigned VOX_INVALID = d->voverflow ? 0u : (unsigned)d->vdiv[0] * (unsigned)d->vdiv[1] * (unsigned)d->vdiv[2];
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
     const unsigned k = keys[i];
     if (k == VOX_INVALID) { slot_of_point[perm[i]] = -1; continue; }
@@ -393,16 +419,7 @@ __global__ void __launch_bounds__(VF_THREADS, 1) vox_fused_kernel(VoxFusedArgs a
       int over = 0;
       unsigned long long cells = 1ull;
       if (finite > 0) {
-        const long long dx = (long long)(__fmul_rn(__fsub_rn(mx[0], mn[0]), a.inv)) + 1;
-        const long long dy = (long long)(__fmul_rn(__fsub_rn(mx[1], mn[1]), a.inv)) + 1;
-        const long long dz = (long long)(__fmul_rn(__fsub_rn(mx[2], mn[2]), a.inv)) + 1;
-        over = (dx * dy * dz > 2147483647ll) ? 1 : 0;
-        for (int c = 0; c < 3; c++) {
-          const int mnb = (int)floorf(__fmul_rn(mn[c], a.inv));
-          const int mxb = (int)floorf(__fmul_rn(mx[c], a.inv));
-          S.minb[c] = mnb;
-          S.div[c] = mxb - mnb + 1;
-        }
+        over = vox_grid_setup(mn, mx, a.inv, S.minb, S.div);
         cells = (unsigned long long)S.div[0] * (unsigned long long)S.div[1] * (unsigned long long)S.div[2];
       } else {
         for (int c = 0; c < 3; c++) { S.minb[c] = 0; S.div[c] = 1; }
@@ -431,7 +448,7 @@ __global__ void __launch_bounds__(VF_THREADS, 1) vox_fused_kernel(VoxFusedArgs a
   // ---- voxel keys of the own chunk (vox_keys_kernel's arithmetic) ----
   {
     const int m0 = S.minb[0], m1 = S.minb[1], m2 = S.minb[2];
-    const int mul1 = S.div[0], mul2 = S.div[0] * S.div[1];
+    const unsigned mul1 = (unsigned)S.div[0], mul2 = (unsigned)S.div[0] * (unsigned)S.div[1];
     for (int j = tid; j < cnt; j += VF_THREADS) {
       const float4 p = a.pts[lo + j];
       unsigned key = S.invalid;
@@ -439,7 +456,7 @@ __global__ void __launch_bounds__(VF_THREADS, 1) vox_fused_kernel(VoxFusedArgs a
         const int i0 = (int)(__fsub_rn(floorf(__fmul_rn(p.x, a.inv)), (float)m0));
         const int i1 = (int)(__fsub_rn(floorf(__fmul_rn(p.y, a.inv)), (float)m1));
         const int i2 = (int)(__fsub_rn(floorf(__fmul_rn(p.z, a.inv)), (float)m2));
-        key = (unsigned)(i0 + i1 * mul1 + i2 * mul2);
+        key = (unsigned)i0 + (unsigned)i1 * mul1 + (unsigned)i2 * mul2;   // < div_b product < 2^32 (vox_grid_setup)
       }
       S.key[j] = key;
       S.val[j] = (unsigned)(lo + j);

@@ -8,7 +8,8 @@
 // What it follows (all paths relative to /root/reference):
 //   voxel filter      pcl::VoxelGrid<PointXYZI>::applyFilter (PCL >=1.10, NOT in the tree; call
 //                     sites src/dlo/odom.cc:460-463,487-490,1160-1163) — restated from the published
-//                     algorithm, see SURVEY.md App. B1
+//                     algorithm, see SURVEY.md App. B1; where PCL's index arithmetic is undefined or wraps
+//                     (voxel_grid_setup) the cloud passes through, as in the GPU kernels
 //   kd-tree           include/nano_gicp/impl/nanoflann_impl.hpp:867-1012 (build), :1230-1250,
 //                     :1355-1418 (query), :149-214 (result set), :441-449 (metric);
 //                     wrapper include/nano_gicp/nanoflann.hpp:113-152 (leaf size 100, int index)
@@ -910,8 +911,36 @@ struct Gicp {
 // ------------------------------------------------------------------------------------------
 // pcl::VoxelGrid<PointXYZI>::applyFilter restated (SURVEY App. B1).  Within-voxel accumulation
 // order is fixed to ascending input index (PCL's own sort is unstable => implementation-defined).
+// Voxel indices are sorted as PCL's cloud_point_index_idx::idx is: unsigned int.
 // returns 0 ok, 1 = index would overflow int32 (PCL warns and passes the input through)
+//
+// Deviation from PCL: its guard only tests dx*dy*dz > INT32_MAX, in int64 that can itself wrap.  Here (and in the
+// GPU kernels, csrc/voxel.cu vox_grid_setup) the cloud also passes through where PCL's arithmetic is undefined or
+// wraps distinct voxels together: an axis extent (max - min) * inv that is not finite or >= 2^31; floor(min * inv) or
+// floor(max * inv) outside int32, or div_b beyond INT32_MAX; floor(max * inv) - (float)min_b rounding past
+// max_b - min_b; a div_b product >= 2^32.  Everywhere else the result is PCL's.
 // ------------------------------------------------------------------------------------------
+static int voxel_grid_setup(const float mn[3], const float mx[3], float inv, int min_b[3], int div_b[3]) {
+  int64_t dxyz = 1;
+  uint64_t cells = 1;
+  for (int d = 0; d < 3; d++) {
+    const float ext = (mx[d] - mn[d]) * inv;
+    if (!(ext < 2147483648.f)) return 1;
+    dxyz *= (int64_t)ext + 1;
+    if (dxyz > (int64_t)INT32_MAX) return 1;
+    const float flo = std::floor(mn[d] * inv), fhi = std::floor(mx[d] * inv);
+    if (!(flo >= -2147483648.f) || !(fhi < 2147483648.f)) return 1;
+    const int64_t span = (int64_t)fhi - (int64_t)flo;
+    const float fspan = fhi - flo;
+    if (span >= (int64_t)INT32_MAX || (int64_t)fspan > span) return 1;
+    cells *= (uint64_t)(span + 1);
+    if (cells >= (1ull << 32)) return 1;
+    min_b[d] = (int)flo;
+    div_b[d] = (int)(span + 1);
+  }
+  return 0;
+}
+
 static int voxel_filter(const float* pts, size_t n, size_t stride, float leaf, float* out, size_t* m_out,
                         int* voxel_of_point /* optional, n ints: output slot per input point, -1 if skipped */) {
   float mn[3] = {FLT_MAX, FLT_MAX, FLT_MAX}, mx[3] = {-FLT_MAX, -FLT_MAX, -FLT_MAX};
@@ -924,16 +953,14 @@ static int voxel_filter(const float* pts, size_t n, size_t stride, float leaf, f
   }
   if (finite == 0) { *m_out = 0; return 0; }
   const float inv = 1.0f / leaf;
-  int64_t dx = (int64_t)((mx[0] - mn[0]) * inv) + 1, dy = (int64_t)((mx[1] - mn[1]) * inv) + 1, dz = (int64_t)((mx[2] - mn[2]) * inv) + 1;
-  if (dx * dy * dz > (int64_t)INT32_MAX) {
+  int min_b[3], div_b[3];
+  if (voxel_grid_setup(mn, mx, inv, min_b, div_b)) {
     for (size_t i = 0; i < n; i++) std::memcpy(out + i * 8, pts + i * stride, 32);
     *m_out = n;
     return 1;
   }
-  int min_b[3], max_b[3], div_b[3];
-  for (int d = 0; d < 3; d++) { min_b[d] = (int)std::floor(mn[d] * inv); max_b[d] = (int)std::floor(mx[d] * inv); div_b[d] = max_b[d] - min_b[d] + 1; }
-  const int mul0 = 1, mul1 = div_b[0], mul2 = div_b[0] * div_b[1];
-  struct Rec { int idx; int pt; };
+  const uint32_t mul0 = 1, mul1 = (uint32_t)div_b[0], mul2 = (uint32_t)div_b[0] * (uint32_t)div_b[1];
+  struct Rec { uint32_t idx; int pt; };
   std::vector<Rec> recs;
   recs.reserve(n);
   for (size_t i = 0; i < n; i++) {
@@ -942,7 +969,7 @@ static int voxel_filter(const float* pts, size_t n, size_t stride, float leaf, f
     int i0 = (int)(std::floor(p[0] * inv) - (float)min_b[0]);
     int i1 = (int)(std::floor(p[1] * inv) - (float)min_b[1]);
     int i2 = (int)(std::floor(p[2] * inv) - (float)min_b[2]);
-    recs.push_back(Rec{i0 * mul0 + i1 * mul1 + i2 * mul2, (int)i});
+    recs.push_back(Rec{(uint32_t)i0 * mul0 + (uint32_t)i1 * mul1 + (uint32_t)i2 * mul2, (int)i});
   }
   std::stable_sort(recs.begin(), recs.end(), [](const Rec& a, const Rec& b) { return a.idx < b.idx; });
   if (voxel_of_point) for (size_t i = 0; i < n; i++) voxel_of_point[i] = -1;
